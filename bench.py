@@ -57,6 +57,8 @@ def parse():
                     help="device-resident leg through the separate stage calls on one stream instead of world_b200_analyze_batch")
     ap.add_argument("--slices", type=int, default=1,
                     help="utterance slices per step: F0 of slice s+1 overlaps CheapTrick/D4C of slice s on a second stream")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step computed (rank 0) to DIR/<name>.npy, float64, for comparing builds")
     a = ap.parse_args()
     if a.config == 2:
         a.f0, a.utts, a.seconds, a.fs = "dio", 1024, 10.0, 16000
@@ -180,6 +182,36 @@ class ClockSampler:
         sm.sort()
         return {"sm_mhz": sm[len(sm) // 2] if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "reasons": sorted(reasons), "samples": len(sm)}
+
+
+def dump_outputs(d, arrays, budget=60_000_000, seed=0):
+    """arrays: name -> [U, L, ...] tensor of one step (L frames).  The f0 contours of every utterance (if they take at
+    most half the budget); of every array, the same fixed seeded sample of utterance rows, as many as fit in what is
+    left, and where not even one row fits, of that row a fixed seeded sample of frames (first and last included).
+    The row and frame indices go to rows.npy and frames.npy.  Returns them."""
+    import numpy as np
+    import torch
+    os.makedirs(d, exist_ok=True)
+    U, L = arrays["f0"].shape
+    full_f0 = arrays["f0"].numel() * 8 <= budget // 2
+    left = budget - (arrays["f0"].numel() * 8 if full_f0 else 0)
+    per_frame = sum(a[0, 0].numel() * 8 for a in arrays.values())
+    rng = np.random.default_rng(seed)
+    k = max(1, min(U, left // (per_frame * L)))
+    rows = np.sort(rng.choice(U, size=k, replace=False))
+    frames = np.arange(L)
+    if left < per_frame * L:
+        inner = rng.choice(np.arange(1, L - 1), size=max(0, left // per_frame - 2), replace=False)
+        frames = np.sort(np.concatenate([[0, L - 1], inner]))
+    dev = arrays["f0"].device
+    ri, fi = torch.as_tensor(rows, device=dev), torch.as_tensor(frames, device=dev)
+    for name, a in arrays.items():
+        np.save(os.path.join(d, name + ".npy"), a.index_select(0, ri).index_select(1, fi).double().cpu().numpy())
+    if full_f0:
+        np.save(os.path.join(d, "f0_all.npy"), arrays["f0"].double().cpu().numpy())
+    np.save(os.path.join(d, "rows.npy"), rows.astype(np.float64))
+    np.save(os.path.join(d, "frames.npy"), frames.astype(np.float64))
+    return {"rows": rows.tolist(), "frames": int(len(frames)), "frames_of": int(L)}
 
 
 def frames_of(fs, n_samples, frame_period=5.0):
@@ -500,6 +532,10 @@ def main():
     prof = w.profile_report()
     clocks = sampler.stop() if rank == 0 else None
     w.synchronize()
+    dumped = None
+    if a.dump_outputs and rank == 0:   # what a caller of the timed path receives from its last step
+        dumped = dump_outputs(a.dump_outputs, {"time_axis": t_fix if spectral else t_loc, "f0": f0_fix if spectral else f0_loc,
+                                               "spectrogram": sp, "aperiodicity": ap})
     if world > 1:
         tms = torch.tensor([ms], dtype=torch.float64, device=dev)
         dist.all_reduce(tms, op=dist.ReduceOp.MAX)
@@ -753,6 +789,8 @@ def main():
            "device_resident_api": ("world_b200_analyze_batch (utterance slices on two internal streams; per-kernel times below overlap, "
                                    "their sum exceeds the step)" if use_lanes else "separate *_batch stage calls on one stream"), "gpu_launches": int(launches), "roofline": roof, "fp64": fp64, "cpu_baseline": cpu,
            "parity": parity, "kernels": kernels}
+    if dumped is not None:
+        out["dumped"] = dumped
     print(json.dumps(out), flush=True)
     if world > 1:
         dist.destroy_process_group()

@@ -38,22 +38,44 @@ def pytest_collection_modifyitems(config, items):
             it.add_marker(skip)
 
 
-@pytest.fixture(scope="session")
-def ref():
-    """The unmodified reference compiled into oracle/_ref (prebuilt file travels to the GPU box)."""
+@pytest.fixture
+def ref(request):
+    """The unmodified reference's results for this test, replayed from tests/golden/reference; with WB_REF_RECORD
+    set, the reference compiled into oracle/_ref runs and its results are stored (tests/refreplay.py)."""
+    import refreplay
+    record = os.environ.get("WB_REF_RECORD")
+    if not record:
+        return refreplay.Replayer(request.node)
     from refworld import RefWorld, REF_LIB
     if not os.path.exists(REF_LIB):
-        if os.path.isdir("/root/reference/src"):
-            subprocess.check_call(["make", "-C", os.path.join(ROOT, "oracle"), "ref"])
-        else:
-            pytest.skip("oracle/_ref/libworld_ref.so missing and /root/reference absent")
-    return RefWorld(REF_LIB)
+        subprocess.check_call(["make", "-C", os.path.join(ROOT, "oracle"), "ref"])
+    rec = refreplay.Recorder(RefWorld(REF_LIB), request.node,
+                             refreplay.GOLDEN_DIR if record == "1" else os.path.abspath(record))
+    request.addfinalizer(rec.save)
+    return rec
+
+
+@pytest.fixture
+def ref_digests(request):
+    """SHA-256 of the reference's results for the tests that compare bytes or bits with it (tests/refreplay.py);
+    with WB_REF_RECORD set they are computed by the compiled reference (.live) and stored."""
+    import refreplay
+    record = os.environ.get("WB_REF_RECORD")
+    if not record:
+        return refreplay.Digests(request.node)
+    from refworld import RefWorld, REF_LIB
+    if not os.path.exists(REF_LIB):
+        subprocess.check_call(["make", "-C", os.path.join(ROOT, "oracle"), "ref"])
+    d = refreplay.Digests(request.node, RefWorld(REF_LIB),
+                          refreplay.GOLDEN_DIR if record == "1" else os.path.abspath(record))
+    request.addfinalizer(d.save)
+    return d
 
 
 @pytest.fixture(scope="session")
 def golden():
-    import numpy as np
-    return np.load(os.path.join(ROOT, "tests", "golden", "vaiueo2d.npz"))
+    import refreplay
+    return refreplay.load_vaiueo2d()
 
 
 @pytest.fixture(scope="session")

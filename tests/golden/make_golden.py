@@ -1,4 +1,4 @@
-"""Generates tests/golden/vaiueo2d.npz from the UNMODIFIED reference (oracle/_ref, built from
+"""Generates tests/golden/vaiueo2d{,_sp,_ap}.npz from the UNMODIFIED reference (oracle/_ref, built from
 /root/reference with the reference's own flags) on the reference's only fixture,
 test/vaiueo2d.wav.  Run in the build container:  python tests/golden/make_golden.py
 The reference ships no expected outputs (SURVEY.md 4), so these vectors are what pins parity."""
@@ -61,9 +61,11 @@ def main():
     # the fixture through the reference's own wavread must be what read_wav() gives
     xr, fsr, nbit = ref.wavread(WAV)
     assert fsr == fs and nbit == 16 and np.array_equal(xr, x)
-    path = os.path.join(ROOT, "tests", "golden", "vaiueo2d.npz")
-    np.savez_compressed(path, **out)
-    print("wrote", path, os.path.getsize(path), "bytes")
+    # the full-size envelope and aperiodicity go to files of their own: every file stays below 1 MB
+    for part, keys in (("_sp", ["sp"]), ("_ap", ["ap"]), ("", [k for k in out if k not in ("sp", "ap")])):
+        path = os.path.join(ROOT, "tests", "golden", f"vaiueo2d{part}.npz")
+        np.savez_compressed(path, **{k: out[k] for k in keys})
+        print("wrote", path, os.path.getsize(path), "bytes")
 
 
 if __name__ == "__main__":

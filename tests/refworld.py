@@ -157,6 +157,13 @@ class RefWorld:
     def decode_spectral_envelope(self, coded, fs, fft_size, dims):
         return self._codec(self.lib.DecodeSpectralEnvelope, coded, fft_size // 2 + 1, fs, fft_size, dims)
 
+    def decimate(self, x, r):
+        """the reference's decimate() (matlabfunctions.cpp)"""
+        x = np.ascontiguousarray(x, dtype=np.float64)
+        y = np.zeros(len(x))
+        self.lib.decimate(x.ctypes.data_as(C.c_void_p), len(x), r, y.ctypes.data_as(C.c_void_p))
+        return y
+
     def wavread(self, path):
         """the reference's own wavread (tools/audioio.cpp:217-252); only in oracle/_ref"""
         self.lib.GetAudioLength.restype = C.c_int
@@ -170,10 +177,12 @@ class RefWorld:
 
 
 def rel_err(got, want, floor=0.0):
-    """max |got-want| / max(|want|, floor); exact zeros in `want` must be matched exactly unless floor>0."""
-    got = np.asarray(got, dtype=np.float64); want = np.asarray(want, dtype=np.float64)
+    """max |got-want| / max(|want|, floor); exact zeros in `want` must be matched exactly unless floor>0.
+    A masked `want` (a sampled stored result, tests/refreplay.py) is compared on its unmasked entries only."""
+    known = ~np.ma.getmaskarray(want)
+    got = np.asarray(got, dtype=np.float64); want = np.ma.getdata(want).astype(np.float64)
     den = np.maximum(np.abs(want), floor)
     diff = np.abs(got - want)
     with np.errstate(divide="ignore", invalid="ignore"):
         r = np.where(den > 0, diff / den, np.where(diff == 0, 0.0, np.inf))
-    return r
+    return np.where(known, r, 0.0)

@@ -131,8 +131,9 @@ def test_gpu_synthesis(gpu_world, ref, golden):
 def test_gpu_legacy_synthesis(gpu_world, ref, golden):
     import ctypes as C
     x, fs = pc.wav_from_golden(golden)
-    f0 = np.ascontiguousarray(golden["f0_harvest"]); t = golden["time_axis"]
-    sp = ref.cheaptrick(x, fs, t, f0); ap = ref.d4c(x, fs, t, f0, 1024)
+    # the reference's own CheapTrick / D4C rows of the DIO path (the stored vectors) as the parameters
+    f0 = np.ascontiguousarray(golden["f0_stonemask"])
+    sp = np.ascontiguousarray(golden["sp"]); ap = np.ascontiguousarray(golden["ap"])
     y = np.zeros(len(x))
     rows_s = (C.c_void_p * len(f0))(*[sp[i].ctypes.data for i in range(len(f0))])
     rows_a = (C.c_void_p * len(f0))(*[ap[i].ctypes.data for i in range(len(f0))])

@@ -33,8 +33,19 @@ def bind(L):
     return L
 
 
-def test_helpers_are_bit_identical_to_the_reference(lib, ref):
-    A, B = bind(lib), bind(ref.lib)
+def out(fn, n, dtype=np.float64, init=0.0):
+    """a fresh output buffer, filled by fn"""
+    o = np.full(n, init, dtype=dtype)
+    fn(o)
+    return o
+
+
+def test_helpers_are_bit_identical_to_the_reference(lib, ref_digests):
+    """Every result is compared with the reference's own for the same input, through the SHA-256 of its bytes
+    (tests/refreplay.py Digests)."""
+    A = bind(lib)
+    B = bind(ref_digests.live.lib) if ref_digests.live is not None else None
+    chk = ref_digests.check
     rng = np.random.default_rng(7)
     for trial in range(200):
         nx = int(rng.integers(2, 40))
@@ -47,33 +58,37 @@ def test_helpers_are_bit_identical_to_the_reference(lib, ref):
         xi = np.sort(rng.uniform(lo, hi, size=ne)).copy()
         if trial % 5 == 0:
             xi = np.sort(np.round(xi * 2) / 2).copy()
-        ia = np.zeros(ne, dtype=np.int32); ib = np.zeros(ne, dtype=np.int32)
-        A.histc(ptr(x), nx, ptr(xi), ne, ptr(ia)); B.histc(ptr(x), nx, ptr(xi), ne, ptr(ib))
-        assert np.array_equal(ia, ib), (trial, x, xi, ia, ib)
-        ya = np.zeros(ne); yb = np.zeros(ne)
-        A.interp1(ptr(x), ptr(y), nx, ptr(xi), ne, ptr(ya)); B.interp1(ptr(x), ptr(y), nx, ptr(xi), ne, ptr(yb))
-        assert np.array_equal(ya, yb)
+        ia = out(lambda o: A.histc(ptr(x), nx, ptr(xi), ne, ptr(o)), ne, np.int32)
+        chk(f"histc {trial}", ia, lambda: out(lambda o: B.histc(ptr(x), nx, ptr(xi), ne, ptr(o)), ne, np.int32))
+        ya = out(lambda o: A.interp1(ptr(x), ptr(y), nx, ptr(xi), ne, ptr(o)), ne)
+        chk(f"interp1 {trial}", ya, lambda: out(lambda o: B.interp1(ptr(x), ptr(y), nx, ptr(xi), ne, ptr(o)), ne))
         # interp1Q inside the grid
         x0, dx = float(rng.normal()), float(rng.uniform(0.1, 2.0))
         q = np.sort(rng.uniform(x0, x0 + dx * (nx - 1), size=ne)).copy()
-        A.interp1Q(x0, dx, ptr(y), nx, ptr(q), ne, ptr(ya)); B.interp1Q(x0, dx, ptr(y), nx, ptr(q), ne, ptr(yb))
-        assert np.array_equal(ya, yb)
-        da = np.zeros(nx); db = np.zeros(nx)
-        A.diff(ptr(y), nx, ptr(da)); B.diff(ptr(y), nx, ptr(db))
-        assert np.array_equal(da, db)
-        assert A.matlab_std(ptr(y), nx) == B.matlab_std(ptr(y), nx)
+        ya = out(lambda o: A.interp1Q(x0, dx, ptr(y), nx, ptr(q), ne, ptr(o)), ne)
+        chk(f"interp1Q {trial}", ya, lambda: out(lambda o: B.interp1Q(x0, dx, ptr(y), nx, ptr(q), ne, ptr(o)), ne))
+        da = out(lambda o: A.diff(ptr(y), nx, ptr(o)), nx)
+        chk(f"diff {trial}", da, lambda: out(lambda o: B.diff(ptr(y), nx, ptr(o)), nx))
+        chk(f"matlab_std {trial}", np.float64(A.matlab_std(ptr(y), nx)), lambda: np.float64(B.matlab_std(ptr(y), nx)))
         v = float(rng.normal() * 100)
-        assert A.matlab_round(v) == B.matlab_round(v) and A.matlab_round(0.5) == 1 and A.matlab_round(-0.5) == -1
+        chk(f"matlab_round {trial}", np.int64(A.matlab_round(v)), lambda: np.int64(B.matlab_round(v)))
+        assert A.matlab_round(0.5) == 1 and A.matlab_round(-0.5) == -1
         n2 = 2 * int(rng.integers(1, 30))
-        z = rng.normal(size=n2); za = np.zeros(n2); zb = np.zeros(n2)
-        A.fftshift(ptr(z), n2, ptr(za)); B.fftshift(ptr(z), n2, ptr(zb))
-        assert np.array_equal(za, zb)
+        z = rng.normal(size=n2)
+        za = out(lambda o: A.fftshift(ptr(z), n2, ptr(o)), n2)
+        chk(f"fftshift {trial}", za, lambda: out(lambda o: B.fftshift(ptr(z), n2, ptr(o)), n2))
     for r in range(1, 14):                                            # 1 and 13: the all-zero default branch
         n = int(rng.integers(40, 3000))
         x = rng.normal(size=n)
-        ya = np.full(n + 16, np.nan); yb = np.full(n + 16, np.nan)
-        A.decimate(ptr(x), n, r, ptr(ya)); B.decimate(ptr(x), n, r, ptr(yb))
-        assert np.array_equal(np.isnan(ya), np.isnan(yb)) and np.array_equal(ya[~np.isnan(ya)], yb[~np.isnan(yb)]), r
-    sa = (C.c_uint32 * 4)(); sb = (C.c_uint32 * 4)()
-    A.randn_reseed(sa); B.randn_reseed(sb)
-    assert [A.randn(sa) for _ in range(1000)] == [B.randn(sb) for _ in range(1000)] and list(sa) == list(sb)
+        # NaN-initialised: which samples are written is part of the result (NaN bytes compare like any others)
+        ya = np.full(n + 16, np.nan); A.decimate(ptr(x), n, r, ptr(ya))
+        chk(f"decimate {r}", ya, lambda: out(lambda o: B.decimate(ptr(x), n, r, ptr(o)), n + 16, init=np.nan))
+    sa = (C.c_uint32 * 4)()
+    A.randn_reseed(sa)
+    ra = np.array([A.randn(sa) for _ in range(1000)] + list(sa), dtype=np.float64)
+
+    def theirs():
+        sb = (C.c_uint32 * 4)()
+        B.randn_reseed(sb)
+        return np.array([B.randn(sb) for _ in range(1000)] + list(sb), dtype=np.float64)
+    chk("randn 1000 draws and state", ra, theirs)

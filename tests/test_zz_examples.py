@@ -20,14 +20,9 @@ NAMES = ["f0analysis", "spanalysis", "apanalysis", "readandsynthesis", "analysis
 
 @pytest.fixture(scope="module")
 def examples():
-    if os.path.isdir("/root/reference/examples"):
-        import __graft_entry__
-        from world_b200 import api
-        if not os.path.exists(api.DEFAULT_LIB):
-            __graft_entry__.build()
-        subprocess.check_call(["make", "-s", "-C", os.path.join(ROOT, "oracle"), "examples"], stdout=subprocess.DEVNULL)
+    # the programs' sources are the reference's, so build() can only compile them where those sources are present
     if not all(os.path.exists(os.path.join(EX, f"{k}_{n}")) for k in ("ref", "b200") for n in NAMES):
-        pytest.skip("oracle/_ref/examples missing and /root/reference absent")
+        pytest.skip("oracle/_ref/examples not built (the reference's example sources were absent at build time)")
     return EX
 
 
